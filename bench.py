@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- shuffled rows/sec of the shuffle hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4] [--dump-outputs DIR]
 
 A "step" is one pass of the shuffle hot path over one batch of synthetic input: map-side hash-partition ->
 exchange (NVLink peer push / NCCL alltoallv when N>1) -> reduce-side merge (reduceByKey) or ordered group
@@ -18,6 +18,9 @@ exchange (NVLink peer push / NCCL alltoallv when N>1) -> reduce-side merge (redu
 Before the timed loop EVERY run (any N, any config) compares one full reduce partition per rank with the oracle
 (oracle/ C restatement) evaluated on that partition's rows gathered from all ranks' inputs, and aborts on a mismatch
 (`parity` in the JSON line).
+
+--dump-outputs DIR writes the result of the last timed step (dump_outputs).  The inputs come from fixed seeds, so two
+builds run with the same arguments can be compared output for output.
 
 --impl reference times the reference's own CPU implementation on the host cores: the UNMODIFIED douban/dpark built
 into baseline/_ref (oracle/build_reference.py) driven through DparkContext('process') by oracle/ref_runner.py;
@@ -94,7 +97,13 @@ def parse():
     ap.add_argument("--exchange", default="push", choices=["push", "fused", "peer", "nccl"],
                     help="N>1: push = local scatter, then one kernel pushing each peer's block over NVLink; "
                          "fused (alias peer) = the scatter kernel stores into peer memory; nccl = alltoallv")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step returned "
+                    "as DIR/<name>.npy (float64, rows in key order, a seeded sample above DUMP_ROWS rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's results (--impl ours)")
     cfg = CONFIGS[args.config]
     args.rows_per_gpu = args.rows_per_gpu or cfg["rows"]
     args.parts_per_gpu = args.parts_per_gpu or cfg["parts"]
@@ -474,6 +483,64 @@ def parity_check(args, keys, vals, out, P, world, rank, dev):
             "seconds": round(time.perf_counter() - t0, 1)}
 
 
+DUMP_ROWS = 1 << 20     # rows per array kept by dump_outputs over all ranks: at most 4 x 8 MiB of .npy files
+
+
+def dump_outputs(path, out, group, world, rank, first_part):
+    """Writes one step's result as float64 .npy files under `path` (names prefixed rank<r>_ when N > 1).  Rows are
+    put in key order, which no run-to-run detail of the kernels changes: keys are unique in a reduce result and name
+    one group each in a group result.  Above DUMP_ROWS / N rows a kind is sampled at positions drawn with a fixed seed.
+    Integer keys and values are exact in float64 for every config (all below 2^53).
+
+      reduce: keys, values, partition (global id per row), partition_counts (distinct keys per local partition)
+      group:  keys, group_sizes, partition (per group), partition_counts (groups per local partition), and values:
+              the groups' values concatenated in key order, each group's in the order the step returned them"""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    cap = DUMP_ROWS // world
+    rng = np.random.default_rng(20240611)
+    prefix = "rank%d_" % rank if world > 1 else ""
+
+    def sample(n, dev):
+        if n <= cap:
+            return torch.arange(n, device=dev)
+        return torch.from_numpy(np.sort(rng.choice(n, cap, replace=False))).to(dev)
+
+    def save(name, t):
+        np.save(os.path.join(path, prefix + name + ".npy"), t.cpu().numpy().astype(np.float64))
+
+    if group:
+        gkeys, gstarts, ng, vals, poff = out
+        G = int(ng.item())
+        keys, starts, poff = gkeys[:G], gstarts[:G + 1].to(torch.int64), poff.to(torch.int64)
+        dev = keys.device
+        part = torch.searchsorted(poff, starts[:-1], right=True) - 1
+        order = torch.argsort(keys, stable=True)
+        sizes, src = (starts[1:] - starts[:-1])[order], starts[:-1][order]
+        sel = order[sample(G, dev)]
+        save("keys", keys[sel])
+        save("group_sizes", starts[1:][sel] - starts[:-1][sel])
+        save("partition", part[sel] + first_part)
+        save("partition_counts", torch.bincount(part, minlength=len(poff) - 1))
+        ends = torch.cumsum(sizes, 0)
+        q = sample(int(ends[-1]) if G else 0, dev)
+        g = torch.searchsorted(ends, q, right=True)
+        save("values", vals[src[g] + q - (ends[g] - sizes[g])])
+    else:
+        okeys, ovals, po, cnt = out
+        po_h, cnt_h = po.cpu().tolist(), cnt.cpu().tolist()
+        dev = okeys.device
+        rows = torch.cat([torch.arange(po_h[j], po_h[j] + cnt_h[j], device=dev) for j in range(len(cnt_h))])
+        keys, vals = okeys[rows], ovals[rows]
+        part = torch.repeat_interleave(torch.arange(len(cnt_h), device=dev), cnt.to(torch.int64))
+        sel = torch.argsort(keys, stable=True)[sample(len(rows), dev)]
+        save("keys", keys[sel])
+        save("values", vals[sel])
+        save("partition", part[sel] + first_part)
+        save("partition_counts", cnt)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -619,11 +686,22 @@ def run_ours(args):
     barrier()
     del ex_events[:]
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         step()
+    last = step()
     e1.record()
     barrier()
     nv.prof_enable(False)
+    if args.dump_outputs:
+        try:
+            if pipe is not None:
+                last = peer.merge_part_results(last)
+            dump_outputs(args.dump_outputs, last, group, world, rank, shuffle.owner_blocks(P, world)[rank])
+        except BaseException:      # the clocks sampler is a child process: do not leave it running
+            if clocks:
+                clocks.stop()
+            raise
+    del last
     launches = nv.launch_count() - launches0
     ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:

@@ -147,21 +147,15 @@ def test_split_like_parallelize_matches_reference_split_sizes():
 
 
 def test_oracle_hash_vs_compiled_reference_extension():
-    """oracle/_ref/portable_hash.so is the reference's own Cython source compiled
-    as-is (oracle/Makefile `ref`); skip when it was not built."""
-    import importlib.util
-    import os
-    import random
-    path = os.path.join(os.path.dirname(orc.__file__), "_ref", "portable_hash.so")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref not built")
-    spec = importlib.util.spec_from_file_location("portable_hash", path)
-    ph = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ph)
-    rnd = random.Random(7)
-    xs = [rnd.randint(-2 ** 63, 2 ** 63 - 1) for _ in range(20000)]
-    assert orc.hash_vec(np.array(xs, dtype=np.int64)).tolist() == [ph.portable_hash(x) for x in xs]
-    fs = [rnd.uniform(-1e9, 1e9) for _ in range(5000)] + [rnd.random() * 2.0 ** rnd.randint(-1000, 1000) for _ in range(5000)]
-    assert orc.hash_vec(np.array(fs, dtype=np.float64)).tolist() == [ph.portable_hash(x) for x in fs]
-    bs = [bytes(rnd.randrange(256) for _ in range(rnd.randrange(0, 64))) for _ in range(5000)]
-    assert [orc.portable_hash(b) for b in bs] == [ph.portable_hash(b) for b in bs]
+    """The reference's own Cython portable_hash, compiled as-is, on 35000 seeded ints, floats and byte strings
+    (tests/golden/make_refhash_golden.py): every hash through the stored SHA-256, a stride sample value by value."""
+    from tests.golden.make_refhash_golden import digest, inputs
+    want = load("ref_portable_hash.json")
+    xs = inputs()
+    got = {"ints": orc.hash_vec(np.array(xs["ints"], dtype=np.int64)).tolist(),
+           "floats": orc.hash_vec(np.array(xs["floats"], dtype=np.float64)).tolist(),
+           "bytes": [orc.portable_hash(b) for b in xs["bytes"]]}
+    for kind, w in want.items():
+        assert len(got[kind]) == w["n"], kind
+        assert got[kind][::w["stride"]] == w["sample"], kind
+        assert digest(got[kind]) == w["sha256"], kind
