@@ -100,13 +100,15 @@ template <> struct Acc<int64_t> {
 };
 
 template <> struct Acc<double> {
+    // SUM starts at -0.0, the IEEE additive identity (-0.0 + x == x for every x, +0.0 + -0.0 == +0.0): a key whose
+    // only values are -0.0 keeps -0.0 in the kernels that add every value into a fresh accumulator
     static int64_t identity(int op) {
-        double d = 0.0;
+        double d = -0.0;
         switch (op) {
         case DPK_OP_MIN: d = INFINITY; break;
         case DPK_OP_MAX: d = -INFINITY; break;
         case DPK_OP_PROD: d = 1.0; break;
-        default: d = 0.0;
+        default: d = -0.0;
         }
         int64_t b;
         memcpy(&b, &d, 8);

@@ -67,6 +67,7 @@ def reduce_by_key_bytes(splits, key_kind, P, thresholds, op, dev, res):
     ok, ov, off, cnt = nv.combine(rx.keys, rx.vals, op, P, rx.seg.contiguous(), rx.part_first, rx.nparts,
                                   thresholds, sb, row_hash=h)
     off_h, cnt_h = off.cpu().tolist(), cnt.cpu().tolist()
+    shuffle.check_counts(cnt_h)
     ok_h, ov_h = ok.cpu().numpy(), ov.cpu().numpy()
     raw = data.tobytes()
     offs_l = offsets

@@ -49,4 +49,13 @@ int hc_bucket(const int64_t *h, int64_t n, int32_t P, int32_t sub_bits, int32_t 
     for (int64_t i = 0; i < n; i++) o[i] = f.bucket(h[i]);
     return 0;
 }
+// slot hash of the shared-memory merge tables (k_smem_aggregate2/3) over 64 key bits
+void hc_slot_hash32(const int64_t *kb, int64_t n, uint32_t *o) { for (int64_t i = 0; i < n; i++) o[i] = dpk::slot_hash32((uint64_t)kb[i]); }
+// fine bucket of the reduce side's second-level split inside its first-level bucket: the PartFn mode 5 that
+// dpk_combine builds for 2^sb2 fine buckets under a first level of sub_bits
+void hc_fine_bucket(const int64_t *h, int64_t n, int32_t sub_bits, int32_t sb2, int32_t *o) {
+    dpk::PartFn f{};
+    f.mode = 5; f.P = 1 << sb2; f.shift = 32 - sub_bits - sb2; f.sub_bits = 0;
+    for (int64_t i = 0; i < n; i++) o[i] = f.bucket(h[i]);
+}
 }

@@ -82,7 +82,9 @@ def test_every_reduce_implementation_gives_the_oracle_result(impl, shape):
     rng = np.random.default_rng(77)
     P, sb = 2, 0
     if shape == "distinct_overflow":
-        n = 3_000_000                       # 1 first-level bucket per partition -> ~5.8 k rows per fine bucket
+        # P = 1, one first-level bucket: the second-level split stops at its cap of 1024 fine buckets, so each holds
+        # ~3e6 / 1024 = 2930 distinct keys > 2048 (AG2_CAP, the most one pass of the shared-memory merge can hold)
+        P, n = 1, 3_000_000
         k = rng.permutation(n).astype(np.int64) * 7919 - 10 ** 9
     elif shape == "hot_keys":
         n = 1_000_000
@@ -393,7 +395,8 @@ def test_slot_claim_variants_agree_with_the_oracle(wide, op, vkind):
     """dpk_set_option("agg_wide"): claiming a shared-memory slot and depositing the first value with one
     128-bit CAS (1) or with a 64-bit key CAS followed by an atomic on the accumulator (0) must both give
     the reference's createCombiner/mergeValue result (dpark/rdd.py:303-327) for every op and value kind,
-    with negative values (high half of the 64-bit add) and mostly-distinct as well as repeated keys."""
+    with negative values (high half of the 64-bit add) and mostly-distinct as well as repeated keys.
+    The switch belongs to the round-1 kernel k_smem_aggregate, which runs only with agg_impl = 0."""
     from dpark_b200 import shuffle
     rng = np.random.default_rng(5 + wide)
     n, P = 700_000, 3
@@ -403,11 +406,13 @@ def test_slot_claim_variants_agree_with_the_oracle(wide, op, vkind):
         v = rng.integers(-2 ** 40, 2 ** 40, n, dtype=np.int64)
     else:
         v = rng.standard_normal(n) * 1e6
+    nv().set_option("agg_impl", 0)
     nv().set_option("agg_wide", wide)
     try:
         res = shuffle.reduce_by_key([dev(k[: n // 2]), dev(k[n // 2:])], [dev(v[: n // 2]), dev(v[n // 2:])], P, op)
     finally:
         nv().set_option("agg_wide", 1)
+        nv().set_option("agg_impl", 1)
     want = orc.reduce_by_key([k[: n // 2], k[n // 2:]], [v[: n // 2], v[n // 2:]], P, op)
     for p, gk, gv in res:
         gk, gv = gk.cpu().numpy(), gv.cpu().numpy()
